@@ -3,6 +3,7 @@
 
   python bench.py [--config 2|3|4|5] [--gpus N] [--steps K] [--warmup W]   our arm (sm_100a kernels via the C ABI)
   python bench.py --impl reference [--config ...] ...                      the reference's own CPU path (oracle/_ref)
+  python bench.py ... --dump-outputs DIR     also write what the timed path returned in its last step (see dump_outputs)
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N             one rank per GPU
 
 Workloads (BASELINE.json `configs`; the default is config 2, the one the metric is quoted on at one GPU):
@@ -314,11 +315,58 @@ def time_aligner(pairs, local, steps, warmup):
     ms = e0.elapsed_time(e1) / steps
     b.download()
     b.sync()
-    bad = sum(1 for k in range(taken) if b.fetch(k)[2] != 0)
+    results = [b.fetch(k) for k in range(taken)]
+    bad = sum(1 for r in results if r[2] != 0)
     b.close()
-    return {"pairs": taken, "pairs_per_s": taken / (ms * 1e-3), "gcups_full_matrix_equivalent": cells / (ms * 1e-3) / 1e9,
+    return results, {"pairs": taken, "pairs_per_s": taken / (ms * 1e-3), "gcups_full_matrix_equivalent": cells / (ms * 1e-3) / 1e9,
             "ms_per_launch": ms, "soft_failures": bad, "kernel": "rp_aln_kernel",
             "bound": "integer issue (bit-vector words in registers; HBM sees only sequences and the stored leaf words)"}
+
+
+# ---------------------------------------------------------------------------------------------------------------
+DUMP_CONSENSUS_BYTES = 46 << 20   # consensus rows; with the aligner's sample and the per-item arrays a dump stays < 64 MB
+DUMP_ALIGNER_PAIRS = 300          # config 5: CIGARs of at most this many overlaps (~10 kb spans: < 12 MB as float32)
+
+
+def dump_outputs(path, out, lens, pol, st):
+    """--dump-outputs: what the last timed end-to-end step handed back to its caller (rp_poa_fetch_all of every batch
+    object: consensus bytes, their lengths, the polished flags, the window statuses) as DIR/<name>.npy, so that two builds
+    run with the same arguments (hence the same seeded windows) can be compared output for output.  Consensus rows are the
+    bytes' codes as float32, zero past each window's length.  When the consensus rows would exceed DUMP_CONSENSUS_BYTES, a
+    fixed seeded sample of windows is written; window_index.npy lists the windows written either way.  The windows are
+    rank 0's; the by-reference leg (e2e.by_reference) computes the same consensus and is not dumped."""
+    import numpy as np
+    n, stride = out.shape
+    keep = min(n, DUMP_CONSENSUS_BYTES // (4 * stride))
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    cons = out[idx].astype(np.float32)
+    cons[np.arange(stride)[None, :] >= lens[idx][:, None]] = 0
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("consensus", cons), ("consensus_length", lens[idx].astype(np.float32)),
+                    ("polished", pol[idx].astype(np.float32)), ("status", st[idx].astype(np.float32)),
+                    ("window_index", idx.astype(np.float64))):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def dump_aligner_outputs(path, results):
+    """config 5, --dump-outputs: what the last timed aligner launch handed back (rp_aln_fetch_cigar per overlap) for a
+    fixed seeded sample of DUMP_ALIGNER_PAIRS overlaps (all of them when there are fewer), listed in aln_index.npy:
+    aln_edit_distance.npy and aln_status.npy per overlap, the CIGAR strings' byte codes concatenated in aln_cigar.npy
+    (float32) with aln_cigar_offset.npy marking where each one starts and ends."""
+    import numpy as np
+    n = len(results)
+    idx = np.arange(n) if n <= DUMP_ALIGNER_PAIRS else np.sort(
+        np.random.default_rng(0).choice(n, DUMP_ALIGNER_PAIRS, replace=False))
+    cigars = [results[i][0] for i in idx]
+    offset = np.zeros(len(idx) + 1, np.float64)
+    offset[1:] = np.cumsum([len(c) for c in cigars])
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("aln_cigar", np.frombuffer(b"".join(cigars), np.uint8).astype(np.float32)),
+                    ("aln_cigar_offset", offset),
+                    ("aln_edit_distance", np.asarray([results[i][1] for i in idx], np.float32)),
+                    ("aln_status", np.asarray([results[i][2] for i in idx], np.float32)),
+                    ("aln_index", idx.astype(np.float64))):
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -372,7 +420,12 @@ def main():
     ap.add_argument("--internal-by-reference", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--e2e-batches", type=int, default=2,
                     help="batch objects the end-to-end arm cycles through (racon's -c/--cudapoa-batches)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed end-to-end step (and, config 5, the last aligner launch) returned as "
+                         "DIR/<name>.npy (rank 0's windows)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this project's timed path computed: not available with --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = env_int("RANK", 0)
@@ -403,12 +456,12 @@ def main():
     cfg = CONFIGS[args.config]
     banded = cfg["banded"] if args.banded < 0 else bool(args.banded)
     wl = cfg["wl"]
-    aligner = None
+    aligner = aln_results = None
     meta = {}
     if cfg["shape"] == "frag":
         fw = frag_workload(args, rank)
         ws = fw["windows"]
-        aligner = time_aligner(fw["pairs"], local, args.steps, args.warmup)
+        aln_results, aligner = time_aligner(fw["pairs"], local, args.steps, args.warmup)
         meta = {"reads_per_gpu": fw["reads"], "overlaps_per_gpu": fw["overlaps"], "windows_total": ws.n_windows * world,
                 "window_build_s": fw["init_s"]}
     else:
@@ -551,7 +604,7 @@ def main():
             if got is not None:
                 last["gathered"] = got
             gather.start(out, lens)
-        last["out"], last["lens"] = out, lens
+        last["out"], last["lens"], last["pol"], last["st"] = out, lens, pol, st
 
     # where the host spends a step (wall clock of this rank's calling thread, summed over the timed steps): filling the
     # objects, queueing H2D + kernel + D2H, waiting for a kernel to finish, reading results back, the consensus gather
@@ -611,6 +664,10 @@ def main():
     e2e_ms = 1e3 * (time.perf_counter() - t0)
     if windows.fnv1a64([out[i, :lens[i]].tobytes() for i in range(min(n, 200))]) != int(checksum, 16):
         raise SystemExit("bench.py: end-to-end arm produced a different consensus than the kernel-only arm")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, lens, last["pol"], last["st"])
+        if aln_results is not None:
+            dump_aligner_outputs(args.dump_outputs, aln_results)
     io = objs[0].info()
     io["h2d_bytes"] = sum(b.info()["h2d_bytes"] for b in objs)
     io["d2h_bytes"] = sum(b.info()["d2h_bytes"] for b in objs)

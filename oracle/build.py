@@ -35,6 +35,14 @@ def build_ref_cudapoa():
     return out if os.path.exists(out) else None
 
 
+def build_integration():
+    """The reference's host program compiled for integration/ (objects, the headers integration/ includes, the sample
+    files) -> oracle/_ref/integration."""
+    _make("integration")
+    out = os.path.join(HERE, "_ref", "integration")
+    return out if os.path.isdir(out) else None
+
+
 def build_refpol():
     out = os.path.join(HERE, "_ref", "refpol_dump")
     if os.path.isdir("/root/reference/src"):

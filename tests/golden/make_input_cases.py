@@ -5,8 +5,11 @@ file-format combination the reference's own tests use (test/racon_test.cpp:86-29
   data of (it frees reads no overlap points at), the target names, the filtered overlap table (ids, strand, coordinates)
   and — SAM input, where the alignment comes from the file — the breaking points of every overlap; one CRC-32 per window
   the reference built (layers with qualities and positions), and count / bases / md5 / names+tags of what it polished
-  (scores 3 -5 -4, w 500, q 10, trimming on, unpolished sequences kept).
-Stored in tests/golden/input_cases.npz.  Run in the CPU container:  python tests/golden/make_input_cases.py"""
+  (scores 3 -5 -4, w 500, q 10, trimming on, unpolished sequences kept); and the md5 of what the reference's command
+  line (integration/_build/racon, CPU path, default options) prints for the fastq_paf files.
+The input files are the cut of the reference's sample under tests/golden/sample/ (tests/golden/make_sample_data.py).
+Stored in tests/golden/sample/input_cases.npz.  Run where the reference is built:  python tests/golden/make_input_cases.py"""
+import hashlib
 import os
 import struct
 import subprocess
@@ -19,7 +22,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from tests.util import window_crcs  # noqa: E402
-DATA = "/root/reference/test/data/"
+DATA = os.path.join(ROOT, "tests", "golden", "sample") + os.sep
 
 # name: reads, overlaps, target, fragment correction, error threshold
 CASES = {
@@ -126,7 +129,13 @@ def main():
             out[name + "/bp_off"], out[name + "/bp"] = bp_off, bp
         print(name, "sequences", len(seqs), "with data", sum(1 for _, d, _ in seqs if d), "overlaps", len(ov), "windows",
               len(wp["window_crc"]), "polished", wp["polished_count"], wp["polished_bases"], wp["polished_md5"])
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "input_cases.npz")
+    racon = os.path.join(ROOT, "integration", "_build", "racon")
+    reads, overlaps, target, _, _ = CASES["fastq_paf"]
+    cli = subprocess.run([racon, "-t", "4", DATA + reads, DATA + overlaps, DATA + target], stdout=subprocess.PIPE,
+                         stderr=subprocess.DEVNULL, check=True).stdout
+    out["cli_md5"] = np.frombuffer(hashlib.md5(cli).hexdigest().encode(), np.uint8)
+    print("racon stdout", len(cli), "bytes, md5", hashlib.md5(cli).hexdigest())
+    path = DATA + "input_cases.npz"
     np.savez_compressed(path, **out)
     print("wrote", path, os.path.getsize(path), "bytes")
 

@@ -6,8 +6,9 @@ integration/cudaaligner.cpp, run on the reference's own sample files.
   * the reference's CUDA test cases (test/racon_test.cpp:297-507) reach the CPU goldens of test/racon_test.cpp:86-295 —
     the reference's own CUDA build does not (it carries separate goldens: 1385, 1607, 1541, 1661, 4168, 1361, 397185 ...).
 
-The binaries and the sample files are built/copied here (CPU container, where /root/reference exists) into
-integration/_build/, which travels to the GPU box with the repo snapshot."""
+`make -C oracle integration` compiles the reference's part and copies the sample files into oracle/_ref/integration/
+(where the reference's sources exist); `make -C integration` (run by build()) links them with integration/'s own sources
+into integration/_build/.  The tests skip where the reference's part was not built."""
 import hashlib
 import json
 import os
@@ -19,7 +20,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "integration", "_build")
 RACON = os.path.join(BUILD, "racon")
 GOLDENS = os.path.join(BUILD, "racon_goldens")
-DATA = os.path.join(BUILD, "data")
+DATA = os.path.join(ROOT, "oracle", "_ref", "integration", "data")
 
 # racon's stdout on the sample with default scores (SURVEY.md §8c: identical for 1/4/8 threads, SISD and AVX2 builds)
 MD5_DEFAULT = "b0e2a2788440a4982e544e2e9b3bf378"
@@ -42,7 +43,7 @@ CPU_GOLDENS = {
 
 def _need_build():
     if not (os.path.exists(RACON) and os.path.exists(GOLDENS) and os.path.isdir(DATA)):
-        pytest.skip("integration/_build missing: run `make -C integration` where /root/reference exists")
+        pytest.skip("integration/_build missing: needs oracle/_ref/integration, built from the reference's sources")
 
 
 def test_integration_binaries_are_the_reference_host_linked_to_the_product_library():

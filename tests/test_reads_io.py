@@ -1,7 +1,9 @@
 """Input layer of the C++ host layer (racon_b200/csrc/reads_io.*; SURVEY §8 f4): FASTA / FASTQ / PAF / MHAP / SAM files ->
 the state racon::Polisher::initialize holds before it looks for breaking points, against what the UNMODIFIED reference
-held for the same files (tests/golden/input_cases.npz, made by tests/golden/make_input_cases.py from oracle/_ref/refpol_dump).
-Host code only: runs without a GPU.  The sample files are the copies `make -C integration` puts under integration/_build/data."""
+held for the same files (tests/golden/sample/input_cases.npz, made by tests/golden/make_input_cases.py from
+oracle/_ref/refpol_dump).
+Host code only: runs without a GPU.  The files are a cut of the reference's lambda sample, tests/golden/sample/
+(tests/golden/make_sample_data.py)."""
 import gzip
 import os
 import zlib
@@ -13,8 +15,8 @@ from racon_b200 import api
 from tests import util
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DATA = os.path.join(ROOT, "integration", "_build", "data")
-GOLD = os.path.join(ROOT, "tests", "golden", "input_cases.npz")
+DATA = os.path.join(ROOT, "tests", "golden", "sample")
+GOLD = os.path.join(DATA, "input_cases.npz")
 
 CASES = {
     "fastq_paf": ("sample_reads.fastq.gz", "sample_overlaps.paf.gz", "sample_layout.fasta.gz", False, 0.3),
@@ -25,8 +27,6 @@ CASES = {
     "frag_fasta_mhap": ("sample_reads.fasta.gz", "sample_ava_overlaps.mhap.gz", "sample_reads.fasta.gz", True, 0.3),
     "fastq_paf_strict": ("sample_reads.fastq.gz", "sample_overlaps.paf.gz", "sample_layout.fasta.gz", False, 0.05),
 }
-
-pytestmark = pytest.mark.skipif(not os.path.isdir(DATA), reason="integration/_build/data missing (run __graft_entry__.build())")
 
 
 def _open(case):
